@@ -2,7 +2,7 @@
 """bench.py -- spectral path samples/s of the 'direct' (unidirectional PT) hot path on B200.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--scene c2|c1|c3|c4|c4b|c4c|c0|c5] [--spp S]
-                  [--partition samples|tiles] [--no-extras]
+                  [--partition samples|tiles] [--no-extras] [--dump-outputs DIR]
 
 Headline workload (BASELINE.json configs[1], SURVEY 8(d) C2): cornellbox.prc, 500x500, 'direct' integrator depth 6, mjitt
 sampler, 1024 spp, diffuse materials + one area light.  One "step" = one complete render of that configuration
@@ -23,6 +23,11 @@ Our arm prints ONE JSON line:
 Multi-GPU (torchrun, one rank per GPU): scene replicated, films combined by prb_film_reduce_comm (NCCL over NVLink, inside
 the C ABI) in the timed region.  Headline partition: sample ranges (rank r renders iterations [r spp, (r+1) spp) of ONE
 N*spp-sample sequence from a decorrelated RNG map -> weak scaling); --partition tiles: interleaved tiles (strong scaling).
+
+--dump-outputs DIR: after the timed steps of the headline workload, what its last step returned goes to DIR/<name>.npy --
+film_xyz (H, W, 3) and sample_count (H, W) of the last render (float32); for c5 a fixed, seeded sample of 2^19 rays of every
+class from the last timed pass (hit ids as float64, u / v / t and occlusion as float32).  The inputs depend on the arguments
+only, so two builds run with the same arguments can be compared output for output.
 
 --impl reference: the reference's own CPU implementation cannot be built here (Eigen/Embree/TBB/OIIO absent, SURVEY F4), so
 the arm times oracle/ (the CPU restatement, std::thread x all host cores) on a bounded sample of the same workload.  This
@@ -257,9 +262,26 @@ class Job:
             self.dist.destroy_process_group()
 
 
-def render_workload(job, prb, key, spp, steps, warmup, partition, want_e2e=True, want_profile=True, cpu_seconds=0.0, clock_sampler=None):
+DUMP_LIMIT_BYTES = 64 << 20
+DUMP_SAMPLE_RAYS = 1 << 19  # c5: rays of every class kept by --dump-outputs (a fixed, seeded sample of the 4 M-ray passes)
+
+
+def dump_outputs(dump_dir, arrays):
+    """--dump-outputs: the arrays the timed path returned in its last step, one DIR/<name>.npy each (float32 / float64), so that
+    the outputs of two builds of the project can be compared on the same inputs"""
+    import numpy as np
+    total = sum(a.nbytes for a in arrays.values())
+    assert all(a.dtype in (np.float32, np.float64) for a in arrays.values())
+    assert total <= DUMP_LIMIT_BYTES, "dump of %d bytes exceeds %d" % (total, DUMP_LIMIT_BYTES)
+    os.makedirs(dump_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(dump_dir, name + ".npy"), np.ascontiguousarray(a))
+
+
+def render_workload(job, prb, key, spp, steps, warmup, partition, want_e2e=True, want_profile=True, cpu_seconds=0.0, clock_sampler=None, dump_dir=None):
     """times `steps` renders of `spp` iterations of scene `key` on job.world GPUs; returns the dict of numbers of this workload
-    (rank 0; None on the other ranks).  partition: 'samples' (weak) | 'tiles' (strong) | 'single'."""
+    (rank 0; None on the other ranks).  partition: 'samples' (weak) | 'tiles' (strong) | 'single'.  dump_dir: write the film of
+    the last timed render (rank 0 holds the combined film) there."""
     import numpy as np
     torch = job.torch
     from pearray_b200 import multigpu
@@ -332,6 +354,9 @@ def render_workload(job, prb, key, spp, steps, warmup, partition, want_e2e=True,
         dev_ms += step_resident()
     job.barrier()
     wall_ms = 1e3 * (time.perf_counter() - wall0)
+    if dump_dir is not None and rank == 0:
+        xyz, cnt = ctx.film()
+        dump_outputs(dump_dir, {"film_xyz": xyz, "sample_count": cnt.astype(np.float32)})
     dev_ms = job.max_over_ranks(dev_ms)
     rank_ms = None
     if world > 1:
@@ -443,12 +468,13 @@ def verify_tile_partition(job, prb, key, iters):
 
 
 # ----------------------------------------------------------------------------------------------- C5: triangle soup
-def soup_workload(job, prb, args, steps, passes, want_cpu, clock_sampler=None):
+def soup_workload(job, prb, args, steps, passes, want_cpu, clock_sampler=None, dump_dir=None):
     """SURVEY 8(d) C5: synthetic N-triangle soup (default 10 M), 2048x2048 pinhole, jittered passes; three ray classes timed
     separately through prb_trace_closest_device / prb_trace_any_device with the ray streams resident in HBM: primary (coherent
     closest hit), shadow (any hit towards a point light at (0,3,0), tfar = dist - 1e-3) and incoherent (cosine-hemisphere bounce
     from every primary hit, closest hit).  The only configuration that streams the BVH from HBM.  Weak scaling over ranks (every
-    rank traces its own passes against the replicated scene)."""
+    rank traces its own passes against the replicated scene).  dump_dir: write a fixed, seeded sample of the hit buffers of
+    every ray class of rank 0's last timed pass there."""
     import numpy as np
     torch = job.torch
     rank, world, dev = job.rank, job.world, job.dev
@@ -481,14 +507,29 @@ def soup_workload(job, prb, args, steps, passes, want_cpu, clock_sampler=None):
     rays = {"primary": 0, "shadow": 0, "incoherent": 0}
     hits = {"primary": 0, "shadow": 0, "incoherent": 0}
     keep = {}
+    dumped = {}
 
-    def one_pass(p, timed):
+    def dump_hits(cls, count, seed):
+        """a fixed, seeded sample of the rays of one class: the hit columns (ids as float64) or the occlusion flags"""
+        sel = np.sort(np.random.default_rng(seed).choice(count, min(count, DUMP_SAMPLE_RAYS), replace=False))
+        idx = torch.from_numpy(sel).to(dev)
+        if cls == "shadow":
+            dumped["shadow_occluded"] = occ[idx].cpu().numpy().astype(np.float32)
+            return
+        for name, col in (("entity_id", ent), ("primitive_id", prim)):
+            dumped["%s_%s" % (cls, name)] = col[idx].cpu().numpy().view(np.uint32).astype(np.float64)
+        for name, col in (("u", u), ("v", v), ("t", t)):
+            dumped["%s_%s" % (cls, name)] = col[idx].cpu().numpy()
+
+    def one_pass(p, timed, capture=False):
         org, dr, _, _ = ctx.generate_camera_rays([(0, 0, res, res)], p)
         o = soa(torch.from_numpy(org).to(dev)); dd = soa(torch.from_numpy(dr).to(dev))
         torch.cuda.synchronize(dev)
         ctx.trace_closest_device(ptrs(o, dd), n, hitp)
         if timed:
             ms["primary"] += ctx.last_device_ms(); rays["primary"] += n
+        if capture:  # the incoherent trace below reuses these hit buffers
+            dump_hits("primary", n, 1)
         hit = ent != -1
         idx = hit.nonzero().squeeze(1)
         m = int(idx.numel())
@@ -521,6 +562,9 @@ def soup_workload(job, prb, args, steps, passes, want_cpu, clock_sampler=None):
         ctx.trace_closest_device(ptrs(bo, bd, tmin, None), m, hitp)
         if timed:
             ms["incoherent"] += ctx.last_device_ms(); rays["incoherent"] += m; hits["incoherent"] += int((ent[:m] != -1).sum())
+        if capture:
+            dump_hits("shadow", m, 2)
+            dump_hits("incoherent", m, 3)
         if not keep:  # one sample of every class, with the device results, for the oracle cross-check and the e2e / cpu legs
             # a contiguous block of the pass, in ray order: the host-buffer leg traces rays as coherent as the resident leg does (a random
             # subset would time the traversal of shuffled rays, 2-3x slower, instead of the copies around it)
@@ -537,11 +581,13 @@ def soup_workload(job, prb, args, steps, passes, want_cpu, clock_sampler=None):
         clock_sampler.start()
     job.barrier()
     wall0 = time.perf_counter()
-    for _ in range(steps):
+    for s in range(steps):
         for p in range(passes):
-            one_pass(rank * passes + p, True)
+            one_pass(rank * passes + p, True, capture=dump_dir is not None and rank == 0 and s == steps - 1 and p == passes - 1)
     torch.cuda.synchronize(dev)
     wall = time.perf_counter() - wall0
+    if dumped:
+        dump_outputs(dump_dir, dumped)
     if clock_sampler is not None and rank == 0:
         clock_sampler.stop()
     tot_ms_max = job.max_over_ranks(sum(ms.values()))
@@ -638,7 +684,7 @@ def run_ours(args, rank, world, local_rank):
     sampler = ClockSampler(local_rank)
     line = None
     if args.scene == "c5":
-        r = soup_workload(job, prb, args, args.steps, args.passes, want_cpu=(world == 1 and not args.no_cpu), clock_sampler=sampler)
+        r = soup_workload(job, prb, args, args.steps, args.passes, want_cpu=(world == 1 and not args.no_cpu), clock_sampler=sampler, dump_dir=args.dump_outputs)
         if rank == 0:
             line = {"metric": r["metric"], "value": r["value"], "unit": r["unit"], "n_gpus": world, "steps": args.steps, "warmup": args.warmup, "ms_per_step": r["ms_per_step"],
                     "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic", "config": r["config"], "classes": r["classes"],
@@ -648,7 +694,8 @@ def run_ours(args, rank, world, local_rank):
         key = args.scene
         scene_spp = {"c1": 64, "c2": 1024, "c3": 128, "c4": 256, "c4b": 4096, "c4c": 4096, "c0": 128}[key]
         spp = scene_spp if args.spp is None else args.spp
-        r = render_workload(job, prb, key, spp, args.steps, args.warmup, args.partition, cpu_seconds=0.0 if args.no_cpu else 12.0, clock_sampler=sampler)
+        r = render_workload(job, prb, key, spp, args.steps, args.warmup, args.partition, cpu_seconds=0.0 if args.no_cpu else 12.0, clock_sampler=sampler,
+                            dump_dir=args.dump_outputs)
         extras = {}
         if not args.no_extras and key == "c2" and args.spp is None:
             if world == 1:
@@ -716,7 +763,14 @@ def main():
     ap.add_argument("--partition", default="samples", choices=["samples", "tiles"])
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline legs")
     ap.add_argument("--no-extras", action="store_true", help="default run: skip the complex.prc / C5 / strong-scaling legs")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the headline workload returned in its last step as DIR/<name>.npy "
+                         "(film + sample counts; c5: a fixed sample of the hit buffers)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs is not None and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
