@@ -583,6 +583,25 @@ enum { PRB_SHADING_AUTO = -1, PRB_SHADING_SINGLE = 0, PRB_SHADING_STAGED = 1 };
 prb_status prb_set_shading_mode(prb_ctx* ctx, int mode);
 prb_status prb_get_shading_mode(prb_ctx* ctx, int* mode);
 
+/* -- the integrator prb_render_tiles runs.  PRB_INTEGRATOR_DIRECT: the path tracer above (reference direct.cpp).
+ * PRB_INTEGRATOR_AO: ambient occlusion (reference plugins/main/integrators/ao.cpp): per sample the camera ray of 'direct' (same
+ * draws) and its closest hit; a miss adds a zero sample and counts no sample; a hit writes the first-hit AOVs and sample count
+ * like 'direct' and traces sample_count cosine-weighted rays about the (unflipped) shading normal any-hit from the safe-position
+ * origin (tmin 1e-4, counted as shadow rays); the sample's value is 1 - occluded / sample_count, pushed as one fragment with the
+ * MIS weight of a zero-radiance miss (heroFactor / (WavelengthPDF * sum heroFactor)) and importance 1.  Films, tiles, resume,
+ * reductions, stats and timings mean the same as under 'direct'; with profiling on, the primary and occlusion kernels count as
+ * PRB_STAGE_TRACE and the film fold as PRB_STAGE_SHADE.
+ * prb_upload_scene resets the integrator to { PRB_INTEGRATOR_DIRECT, 0 }.  prb_set_integrator fails with PRB_ERR_NO_SCENE before
+ * a scene was uploaded, PRB_ERR_INVALID_ARG for an unknown type or 'ao' with sample_count 0, PRB_ERR_UNSUPPORTED for 'ao' on a
+ * scene with light path expression channels. */
+enum { PRB_INTEGRATOR_DIRECT = 0, PRB_INTEGRATOR_AO = 1 };
+typedef struct prb_integrator {
+	uint32_t type;		   /* PRB_INTEGRATOR_* */
+	uint32_t sample_count; /* AO: occlusion rays per pixel sample (reference parameter 'sample_count', default 10) */
+} prb_integrator;
+prb_status prb_set_integrator(prb_ctx* ctx, const prb_integrator* integrator);
+prb_status prb_get_integrator(prb_ctx* ctx, prb_integrator* out);
+
 #ifdef __cplusplus
 }
 #endif

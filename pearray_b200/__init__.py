@@ -137,6 +137,13 @@ class Stats(C.Structure):
         return int(self.primary_ray_count + self.bounce_ray_count + self.shadow_ray_count)
 
 
+INTEGRATOR = {"direct": 0, "ao": 1}  # PRB_INTEGRATOR_*
+
+
+class Integrator(C.Structure):
+    _fields_ = [("type", C.c_uint32), ("sample_count", C.c_uint32)]
+
+
 class MaterialQuery(C.Structure):
     _fields_ = [("V", C.c_float * 3), ("L", C.c_float * 3), ("wavelength_nm", C.c_float * 4), ("uv", C.c_float * 2),
                 ("ray_flags", C.c_uint32), ("material_id", C.c_uint32), ("rng_state", C.c_uint64)]
@@ -158,7 +165,8 @@ ABI_SYMBOLS = ["prb_create", "prb_destroy", "prb_last_error", "prb_device_count"
                "prb_trace_any", "prb_trace_closest_device", "prb_trace_any_device", "prb_generate_camera_rays",
                "prb_material_eval", "prb_material_sample", "prb_get_stats", "prb_reset_stats", "prb_last_device_ms",
                "prb_set_profiling", "prb_get_stage_times", "prb_film_reduce", "prb_comm_unique_id", "prb_comm_init",
-               "prb_comm_destroy", "prb_film_reduce_comm", "prb_last_reduce_ms", "prb_set_shading_mode", "prb_get_shading_mode", "prb_film_download_lpe", "prb_film_download_aov_ext"]
+               "prb_comm_destroy", "prb_film_reduce_comm", "prb_last_reduce_ms", "prb_set_shading_mode", "prb_get_shading_mode", "prb_film_download_lpe", "prb_film_download_aov_ext",
+               "prb_set_integrator", "prb_get_integrator"]
 
 
 def device_lib():
@@ -208,6 +216,8 @@ def device_lib():
         lib.prb_film_download_aov_ext.argtypes = [C.c_void_p, C.c_void_p]
         lib.prb_set_shading_mode.argtypes = [C.c_void_p, C.c_int]
         lib.prb_get_shading_mode.argtypes = [C.c_void_p, C.POINTER(C.c_int)]
+        lib.prb_set_integrator.argtypes = [C.c_void_p, C.POINTER(Integrator)]
+        lib.prb_get_integrator.argtypes = [C.c_void_p, C.POINTER(Integrator)]
         _dev = lib
     return _dev
 
@@ -231,6 +241,7 @@ def host_lib():
         lib.prh_free_scene.argtypes = [C.c_void_p]
         lib.prh_scene_desc.restype = C.POINTER(SceneDesc)
         lib.prh_scene_desc.argtypes = [C.c_void_p]
+        lib.prh_scene_integrator.argtypes = [C.c_void_p, C.POINTER(Integrator)]
         lib.prh_scene_bvh_seconds.restype = C.c_double
         lib.prh_scene_bvh_seconds.argtypes = [C.c_void_p]
         lib.prh_scene_radius.restype = C.c_float
@@ -310,6 +321,14 @@ class Scene:
     def bvh_build_seconds(self):
         return float(host_lib().prh_scene_bvh_seconds(self._h))
 
+    @property
+    def integrator(self):
+        """the Integrator record of the scene's (integrator ...) block"""
+        rec = Integrator()
+        if host_lib().prh_scene_integrator(self._h, C.byref(rec)) != 0:
+            raise PrbError("prh_scene_integrator: " + host_lib().prh_last_error().decode())
+        return rec
+
     def set_spp(self, spp):
         host_lib().prh_scene_set_spp(self._h, spp)
 
@@ -374,8 +393,25 @@ class Context:
             raise PrbError(what + ": " + self._lib.prb_last_error().decode())
 
     def upload_scene(self, scene):
+        """uploads the scene and selects the integrator of its (integrator ...) block"""
         self._chk(self._lib.prb_upload_scene(self._h, scene.desc), "prb_upload_scene")
         self.scene = scene
+        rec = scene.integrator
+        if rec.type != INTEGRATOR["direct"]:  # 'direct' is what prb_upload_scene leaves selected
+            self.set_integrator(rec.type, rec.sample_count)
+
+    def set_integrator(self, integrator, sample_count=0):
+        """integrator: "direct" / "ao" or a PRB_INTEGRATOR_* value; sample_count: occlusion rays per sample ('ao')"""
+        t = INTEGRATOR[integrator] if isinstance(integrator, str) else int(integrator)
+        rec = Integrator(t, int(sample_count))
+        self._chk(self._lib.prb_set_integrator(self._h, C.byref(rec)), "prb_set_integrator")
+
+    @property
+    def integrator(self):
+        """(type, sample_count) of the integrator prb_render_tiles runs"""
+        rec = Integrator()
+        self._chk(self._lib.prb_get_integrator(self._h, C.byref(rec)), "prb_get_integrator")
+        return int(rec.type), int(rec.sample_count)
 
     def upload_rng(self, states):
         states = np.ascontiguousarray(states, dtype=np.uint64)

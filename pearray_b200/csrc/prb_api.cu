@@ -1,6 +1,6 @@
 // C-ABI implementation (include/prb200_abi.h) over the CUDA kernels.  sm_100a only; no CPU fallback: every
 // entry point fails with PRB_ERR_NO_DEVICE / PRB_ERR_CUDA when no B200-class device is usable.
-#include "dev_wavefront.cuh"
+#include "dev_ao.cuh"
 
 #include <dlfcn.h>
 
@@ -154,6 +154,14 @@ struct prb_ctx {
 	std::vector<cudaEvent_t> profEvents; // pairs
 	float stageMs[PRB_STAGE__COUNT] = {};
 	uint64_t stageLaunches[PRB_STAGE__COUNT] = {};
+	// the integrator prb_render_tiles runs (prb_set_integrator; prb_upload_scene resets it to 'direct')
+	prb_integrator integrator{ PRB_INTEGRATOR_DIRECT, 0 };
+	// 'ao': per-slot state of the running sample, the hit list, the jump-ahead table, and a graph of its own
+	DBuf<uint64_t> aoRng, aoJump;
+	DBuf<uint32_t> aoOccluded, aoHits;
+	int gridAOSmall = 148 * 4, gridAO = 148 * 4; // persistent k_ao_occlusion grids
+	cudaGraphExec_t aoGraph = nullptr;
+	uint64_t aoGraphKey[6] = {};
 };
 
 template <int KIND>
@@ -224,6 +232,10 @@ prb_status prb_create(int device, prb_ctx** out)
 			c->gridTraceClosest = c->smCount * nb;
 		if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k_trace_any, 128, 0) == cudaSuccess && nb > 0)
 			c->gridTraceAny = c->smCount * nb;
+		if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k_ao_occlusion<true>, 128, 0) == cudaSuccess && nb > 0)
+			c->gridAOSmall = c->smCount * nb;
+		if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k_ao_occlusion<false>, 128, 0) == cudaSuccess && nb > 0)
+			c->gridAO = c->smCount * nb;
 	}
 	if (e != cudaSuccess) {
 		delete c;
@@ -242,6 +254,12 @@ void prb_destroy(prb_ctx* c)
 	for (cudaGraphExec_t& g : c->graphExec)
 		if (g)
 			cudaGraphExecDestroy(g);
+	if (c->aoGraph)
+		cudaGraphExecDestroy(c->aoGraph);
+	c->aoRng.release();
+	c->aoJump.release();
+	c->aoOccluded.release();
+	c->aoHits.release();
 	prb_comm_destroy(c);
 	c->reduceF.release();
 	c->reduceU.release();
@@ -681,6 +699,7 @@ prb_status prb_upload_scene(prb_ctx* c, const prb_scene_desc* d)
 	for (uint32_t q = 0; q < c->nQueues; ++q)
 		c->nNeeQueues += c->queueWantsNEE[q] ? 1u : 0u;
 	c->haveScene   = true;
+	c->integrator  = prb_integrator{ PRB_INTEGRATOR_DIRECT, 0 };
 	c->rngUploaded = false; // the RNG map was zeroed above: state 0 of the pcg32_fast MCG stays 0 forever
 	c->cachedTiles.clear();
 	c->nSlots = 0;
@@ -936,6 +955,140 @@ static WFState makeWF(prb_ctx* c, uint32_t first, uint32_t count)
 	return W;
 }
 
+// 'ao': exactly iteration_count iterations of one sample per slot (k_ao_primary, k_ao_occlusion, k_ao_fold), ITERS_PER_GRAPH to a
+// CUDA graph; the kernels of the iterations past the end of the range find every slot done (CNT_END_ITER) and return at once
+static prb_status renderAO(prb_ctx* c, uint32_t first, uint32_t count)
+{
+	constexpr int ITERS_PER_GRAPH = 8;
+	const uint32_t n = c->integrator.sample_count;
+	if ((uint64_t)c->nSlots * n > 0xFFFFFFFFull)
+		return fail(PRB_ERR_UNSUPPORTED, "'ao': owned pixels x sample_count exceeds the 32-bit work counter");
+	CU(c->aoRng.alloc(c->nSlots));
+	CU(c->aoOccluded.alloc(c->nSlots));
+	CU(c->aoHits.alloc(c->nSlots));
+	cudaStream_t s	 = c->stream;
+	const WFState W	 = makeWF(c, first, count);
+	AOState A{ c->aoRng.p, c->aoOccluded.p, c->aoHits.p, c->aoJump.p, n, 0 };
+	const int blocks = (int)((c->nSlots + 127) / 128);
+	c->lastFirstIter = first;
+	c->lastEndIter	 = first + count;
+	auto launch		 = [&](uint32_t parity, int kernel) { // kernel 0: primary, 1: occlusion, 2: fold
+		A.parity = parity;
+		if (kernel == 0) {
+			if (c->smallScene)
+				k_ao_primary<true><<<blocks, 128, 0, s>>>(c->S, W, A);
+			else
+				k_ao_primary<false><<<blocks, 128, 0, s>>>(c->S, W, A);
+		} else if (kernel == 1) {
+			if (c->smallScene)
+				k_ao_occlusion<true><<<c->gridAOSmall, 128, 0, s>>>(c->S, W, A);
+			else
+				k_ao_occlusion<false><<<c->gridAO, 128, 0, s>>>(c->S, W, A);
+		} else {
+			k_ao_fold<<<blocks, 128, 0, s>>>(c->S, W, A);
+		}
+	};
+	CU(cudaEventRecord(c->evA, s));
+	CU(cudaMemsetAsync(c->counters.p, 0, CNT__COUNT * sizeof(uint32_t), s));
+	k_ao_begin<<<blocks, 128, 0, s>>>(W, A);
+	CU(cudaGetLastError());
+	const uint32_t rounds = (count + ITERS_PER_GRAPH - 1) / ITERS_PER_GRAPH;
+	if (c->profiling) { // the same launches without graph replay, each bracketed by an event pair: primary + occlusion TRACE, fold SHADE
+		while (c->profEvents.size() < 6) {
+			cudaEvent_t ev;
+			CU(cudaEventCreate(&ev));
+			c->profEvents.push_back(ev);
+		}
+		for (uint32_t r = 0; r < rounds * ITERS_PER_GRAPH; ++r)
+			for (int k = 0; k < 3; ++k) {
+				CU(cudaEventRecord(c->profEvents[2 * k], s));
+				launch(r & 1u, k);
+				CU(cudaEventRecord(c->profEvents[2 * k + 1], s));
+				CU(cudaGetLastError());
+				CU(cudaEventSynchronize(c->profEvents[2 * k + 1]));
+				float ms = 0;
+				CU(cudaEventElapsedTime(&ms, c->profEvents[2 * k], c->profEvents[2 * k + 1]));
+				const int stage = k == 2 ? PRB_STAGE_SHADE : PRB_STAGE_TRACE;
+				c->stageMs[stage] += ms;
+				c->stageLaunches[stage] += 1;
+			}
+	} else {
+		// the kernels read the iteration range from device memory, so one graph serves every call until the scene, the slot
+		// buffers, the trace variant or sample_count change
+		const uint64_t key[6] = { c->stateVersion, (uint64_t)(c->smallScene ? 1u : 0u) | (c->wantAOV ? 2u : 0u), n,
+								  (uint64_t)(uintptr_t)A.jump, (uint64_t)(uintptr_t)A.rng, (uint64_t)(uintptr_t)A.hits };
+		if (!c->aoGraph || std::memcmp(key, c->aoGraphKey, sizeof(key)) != 0) {
+			if (c->aoGraph) {
+				cudaGraphExecDestroy(c->aoGraph);
+				c->aoGraph = nullptr;
+			}
+			cudaGraph_t graph = nullptr;
+			cudaError_t be	  = cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal);
+			if (be == cudaSuccess)
+				for (int r = 0; r < ITERS_PER_GRAPH; ++r)
+					for (int k = 0; k < 3; ++k)
+						launch((uint32_t)(r & 1), k);
+			const cudaError_t ce = be == cudaSuccess ? cudaGetLastError() : be;
+			const cudaError_t ee = be == cudaSuccess ? cudaStreamEndCapture(s, &graph) : be;
+			if (ce != cudaSuccess || ee != cudaSuccess) {
+				if (graph)
+					cudaGraphDestroy(graph);
+				return fail(PRB_ERR_CUDA, std::string("graph capture failed: ") + cudaGetErrorString(ce != cudaSuccess ? ce : ee));
+			}
+			const cudaError_t ie = cudaGraphInstantiate(&c->aoGraph, graph, 0);
+			cudaGraphDestroy(graph);
+			if (ie != cudaSuccess) {
+				c->aoGraph = nullptr;
+				return fail(PRB_ERR_CUDA, std::string("graph instantiation failed: ") + cudaGetErrorString(ie));
+			}
+			std::memcpy(c->aoGraphKey, key, sizeof(key));
+		}
+		for (uint32_t r = 0; r < rounds; ++r)
+			CU(cudaGraphLaunch(c->aoGraph, s));
+	}
+	c->kernelLaunches += 1 + 3ull * ITERS_PER_GRAPH * rounds;
+	c->wavefrontIterations += (uint64_t)ITERS_PER_GRAPH * rounds;
+	CU(cudaEventRecord(c->evB, s));
+	CU(cudaEventSynchronize(c->evB));
+	CU(cudaEventElapsedTime(&c->lastMs, c->evA, c->evB));
+	return PRB_OK;
+}
+
+prb_status prb_set_integrator(prb_ctx* c, const prb_integrator* in)
+{
+	if (!c || !in)
+		return fail(PRB_ERR_INVALID_ARG, "null argument");
+	if (!c->haveScene)
+		return fail(PRB_ERR_NO_SCENE, "no scene uploaded");
+	if (in->type != PRB_INTEGRATOR_DIRECT && in->type != PRB_INTEGRATOR_AO)
+		return fail(PRB_ERR_INVALID_ARG, "unknown integrator type " + std::to_string(in->type));
+	if (in->type == PRB_INTEGRATOR_AO) {
+		if (in->sample_count == 0)
+			return fail(PRB_ERR_INVALID_ARG, "'ao' needs sample_count >= 1");
+		if (c->S.nLPE)
+			return fail(PRB_ERR_UNSUPPORTED, "'ao' does not fill light path expression channels");
+		// jump[j] = M^(2j) mod 2^64: the pcg32_fast state after the two draws of each of j occlusion rays is s * jump[j]
+		std::vector<uint64_t> jump(in->sample_count + 1);
+		uint64_t m = 1;
+		for (auto& v : jump) {
+			v = m;
+			m *= 6364136223846793005ULL * 6364136223846793005ULL;
+		}
+		CU(cudaSetDevice(c->device));
+		CU(c->aoJump.upload(jump.data(), jump.size(), c->stream));
+		CU(cudaStreamSynchronize(c->stream));
+	}
+	c->integrator = *in;
+	return PRB_OK;
+}
+prb_status prb_get_integrator(prb_ctx* c, prb_integrator* out)
+{
+	if (!c || !out)
+		return fail(PRB_ERR_INVALID_ARG, "null argument");
+	*out = c->integrator;
+	return PRB_OK;
+}
+
 prb_status prb_render_tiles(prb_ctx* c, const prb_tile* tiles, size_t n_tiles, uint32_t first_iteration, uint32_t iteration_count)
 {
 	if (!c || !tiles)
@@ -950,6 +1103,8 @@ prb_status prb_render_tiles(prb_ctx* c, const prb_tile* tiles, size_t n_tiles, u
 	prb_status st = setupSlots(c, tiles, n_tiles);
 	if (st != PRB_OK)
 		return st;
+	if (c->integrator.type == PRB_INTEGRATOR_AO)
+		return renderAO(c, first_iteration, iteration_count);
 	cudaStream_t s = c->stream;
 	const WFState W	 = makeWF(c, first_iteration, iteration_count);
 	const int blocks = (int)((c->nSlots + 127) / 128);

@@ -77,6 +77,7 @@ uint32_t prh_abi_sizeof(const char* name)
 	PRH_SIZE_OF(prb_stats)
 	PRH_SIZE_OF(prb_material_query)
 	PRH_SIZE_OF(prb_material_result)
+	PRH_SIZE_OF(prb_integrator)
 #undef PRH_SIZE_OF
 	return 0;
 }
@@ -143,6 +144,16 @@ int prh_save_outputs(void* h, const char* dir, const float* xyz, const uint32_t*
 }
 void prh_free_scene(void* h) { delete static_cast<SceneHandle*>(h); }
 const prb_scene_desc* prh_scene_desc(void* h) { return &static_cast<SceneHandle*>(h)->scene->desc; }
+// the prb_integrator record of the scene's (integrator ...) block; PRB_ERR_INVALID_ARG for a null argument
+int prh_scene_integrator(void* h, prb_integrator* out)
+{
+	if (!h || !out) {
+		g_err = "null argument";
+		return PRB_ERR_INVALID_ARG;
+	}
+	*out = static_cast<SceneHandle*>(h)->scene->integrator;
+	return PRB_OK;
+}
 prb_scene_desc* prh_scene_desc_mutable(void* h) { return &static_cast<SceneHandle*>(h)->scene->desc; }
 double prh_scene_bvh_seconds(void* h) { return static_cast<SceneHandle*>(h)->scene->bvhBuildSeconds; }
 float prh_scene_radius(void* h) { return static_cast<SceneHandle*>(h)->scene->sceneRadius; }

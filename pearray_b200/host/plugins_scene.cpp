@@ -1216,6 +1216,52 @@ void IntDirectInstance::onTile(RenderTileSession& session)
 		PR_LOG(L_ERROR) << "prb_render_tiles failed: " << prb_last_error() << std::endl;
 }
 
+// ------------------------------------------------------------------ 'ao' integrator -> device
+// reference plugins/main/integrators/ao.cpp: one parameter, sample_count (occlusion rays per pixel sample, default 10).  The
+// tiles go to prb_render_tiles like 'direct'; RenderContext selects the kernels with prb_set_integrator.
+class IntAO : public IIntegrator {
+public:
+	explicit IntAO(uint32 sampleCount)
+		: mSampleCount(sampleCount)
+	{
+	}
+	std::shared_ptr<IIntegratorInstance> createThreadInstance(RenderContext*, size_t) override { return std::make_shared<IntDirectInstance>(); }
+	void describe(prb_settings& s) const override
+	{ // no path beyond the first hit, no light sampling
+		s.max_ray_depth		 = 1;
+		s.soft_max_ray_depth = 1;
+		s.do_nee = s.do_direct = s.emissive_scatter = 0;
+	}
+	prb_integrator deviceIntegrator() const override { return prb_integrator{ PRB_INTEGRATOR_AO, mSampleCount }; }
+
+private:
+	uint32 mSampleCount;
+};
+class IntAOFactory : public IIntegratorFactory {
+public:
+	explicit IntAOFactory(const ParameterGroup& params)
+	{
+		const uint64 n = params.getUInt("sample_count", 10);
+		if (n == 0)
+			PR_LOG(L_ERROR) << "[ao] sample_count must be at least 1; using 1" << std::endl;
+		mSampleCount = (uint32)std::min<uint64>(std::max<uint64>(n, 1), 0xFFFFFFFFu);
+	}
+	std::shared_ptr<IIntegrator> createInstance() const override { return std::make_shared<IntAO>(mSampleCount); }
+
+private:
+	uint32 mSampleCount = 10;
+};
+class IntAOFactoryFactory : public IIntegratorPlugin {
+public:
+	std::shared_ptr<IIntegratorFactory> create(const std::string&, const SceneLoadContext& ctx) override { return std::make_shared<IntAOFactory>(ctx.parameters()); }
+	const std::vector<std::string>& getNames() const override
+	{
+		static const std::vector<std::string> names({ "ao", "ambientocclusion", "occlusion" });
+		return names;
+	}
+	std::string specification(const std::string&) const override { return "AO / Ambient Occlusion: sample_count (10)"; }
+};
+
 void registerScenePlugins(std::vector<std::shared_ptr<IPlugin>>& out)
 {
 	out.push_back(std::make_shared<MeshEntityPlugin>());
@@ -1239,5 +1285,6 @@ void registerScenePlugins(std::vector<std::shared_ptr<IPlugin>>& out)
 	out.push_back(std::make_shared<CIESpectralMapperPlugin>());
 	out.push_back(std::make_shared<AGHSpectralMapperPlugin>());
 	out.push_back(std::make_shared<IntDirectFactoryFactory>());
+	out.push_back(std::make_shared<IntAOFactoryFactory>());
 }
 } // namespace PR

@@ -495,6 +495,8 @@ public:
 	virtual void onEnd() {}
 	virtual std::shared_ptr<IIntegratorInstance> createThreadInstance(RenderContext* ctx, size_t thread_index) = 0;
 	virtual void describe(prb_settings& s) const = 0;
+	// the record prb_set_integrator takes for this integrator (RenderContext applies it after prb_upload_scene)
+	virtual prb_integrator deviceIntegrator() const { return prb_integrator{ PRB_INTEGRATOR_DIRECT, 0 }; }
 };
 class IIntegratorFactory { // reference src/core/integrator/IIntegratorFactory.h:7-12
 public:
@@ -908,6 +910,7 @@ BVH8 buildBVH8(const BVHBuildInput& in, int maxLeafPrims);
 class CompiledScene {
 public:
 	prb_scene_desc desc{};
+	prb_integrator integrator{ PRB_INTEGRATOR_DIRECT, 0 }; // the scene's (integrator ...) block, for prb_set_integrator
 	std::vector<prb_node> nodes;
 	std::vector<prb_material> materials;
 	std::vector<prb_emission> emissions;

@@ -23,6 +23,12 @@ RenderContext::RenderContext(const std::shared_ptr<Environment>& env, int device
 		PR_LOG(L_ERROR) << "prb_upload_scene failed: " << prb_last_error() << std::endl;
 		prb_destroy(mCtx);
 		mCtx = nullptr;
+		return;
+	}
+	if (prb_set_integrator(mCtx, &mScene->integrator) != PRB_OK) {
+		PR_LOG(L_ERROR) << "prb_set_integrator failed: " << prb_last_error() << std::endl;
+		prb_destroy(mCtx);
+		mCtx = nullptr;
 	}
 }
 RenderContext::~RenderContext()

@@ -197,7 +197,11 @@ std::shared_ptr<CompiledScene> SceneCompiler::compile()
 	st.spectral_end			 = rs.spectralEnd;
 	st.time_alpha			 = 1 * rs.timeScale; // TimeMappingMode::Right (RenderSettings.cpp:16, RenderTile.cpp:49-52)
 	st.time_beta			 = 0;
-	rs.integratorFactory->createInstance()->describe(st);
+	{
+		const auto integrator = rs.integratorFactory->createInstance();
+		integrator->describe(st);
+		s.integrator = integrator->deviceIntegrator();
+	}
 	mEnv->activeCamera->describe(s.desc.camera);
 
 	// spectral tables first in the pool
