@@ -591,13 +591,30 @@ prb_status prb_get_shading_mode(prb_ctx* ctx, int* mode);
  * MIS weight of a zero-radiance miss (heroFactor / (WavelengthPDF * sum heroFactor)) and importance 1.  Films, tiles, resume,
  * reductions, stats and timings mean the same as under 'direct'; with profiling on, the primary and occlusion kernels count as
  * PRB_STAGE_TRACE and the film fold as PRB_STAGE_SHADE.
+ * PRB_INTEGRATOR_VF: visual feedback, the debug view of scene set-up (reference plugins/main/integrators/visualfeedback.cpp):
+ * per sample the camera ray of 'direct' (same draws) and its closest hit.  A miss is handled as under 'ao'.  A hit writes the
+ * first-hit AOVs and sample count like 'direct' and one linear-sRGB colour c chosen by `mode` (PRB_VF_*):
+ *   ENTITY_ID palette(entity id)           MATERIAL_ID palette(material id), black for PRB_INVALID_ID
+ *   EMISSION_ID palette(emission id), black for PRB_INVALID_ID    PRIMITIVE_ID palette(face index; 0 for spheres and planes)
+ *   PARAMETER (u, v, 0) of the first-hit AOV   INSIDE (1, 0, 0) when dot(D, N) > 0 (back face), else (0, 1, 0)
+ *   NDOTV |dot(N, D)| (1, 1, 1)            (D: the normalised camera direction, N: the geometry normal of the hit)
+ * palette(id), in fp32: h = frac(id * 0.618034), S = 0.7, V = 0.9, then the textbook HSV -> RGB.  The sample's value is
+ * XYZ = M c with M the sRGB (D65) RGB -> XYZ matrix, folded into the film as it is, without the spectral fragment path (also
+ * on a monotonic film), so the sRGB tone mode of the film gives back c.  The RNG stream ends after the camera draws.  Films,
+ * tiles, resume, reductions, stats and timings mean the same as under 'ao'; with profiling on, its one kernel counts as
+ * PRB_STAGE_TRACE.
  * prb_upload_scene resets the integrator to { PRB_INTEGRATOR_DIRECT, 0 }.  prb_set_integrator fails with PRB_ERR_NO_SCENE before
- * a scene was uploaded, PRB_ERR_INVALID_ARG for an unknown type or 'ao' with sample_count 0, PRB_ERR_UNSUPPORTED for 'ao' on a
- * scene with light path expression channels. */
-enum { PRB_INTEGRATOR_DIRECT = 0, PRB_INTEGRATOR_AO = 1 };
+ * a scene was uploaded, PRB_ERR_INVALID_ARG for an unknown type, 'ao' with sample_count 0 or 'vf' with an unknown mode,
+ * PRB_ERR_UNSUPPORTED for 'ao' or 'vf' on a scene with light path expression channels. */
+enum { PRB_INTEGRATOR_DIRECT = 0, PRB_INTEGRATOR_AO = 1, PRB_INTEGRATOR_VF = 2 };
+enum { PRB_VF_ENTITY_ID, PRB_VF_MATERIAL_ID, PRB_VF_EMISSION_ID, PRB_VF_PRIMITIVE_ID, PRB_VF_PARAMETER, PRB_VF_INSIDE, PRB_VF_NDOTV, PRB_VF__COUNT };
+/* 8 bytes: the parameter of each integrator shares the second word, so records of existing callers keep their size */
 typedef struct prb_integrator {
-	uint32_t type;		   /* PRB_INTEGRATOR_* */
-	uint32_t sample_count; /* AO: occlusion rays per pixel sample (reference parameter 'sample_count', default 10) */
+	uint32_t type; /* PRB_INTEGRATOR_* */
+	union {
+		uint32_t sample_count; /* AO: occlusion rays per pixel sample (reference parameter 'sample_count', default 10) */
+		uint32_t mode;		   /* VF: PRB_VF_* (reference parameter 'mode', default colored_entity_id) */
+	};
 } prb_integrator;
 prb_status prb_set_integrator(prb_ctx* ctx, const prb_integrator* integrator);
 prb_status prb_get_integrator(prb_ctx* ctx, prb_integrator* out);

@@ -137,11 +137,16 @@ class Stats(C.Structure):
         return int(self.primary_ray_count + self.bounce_ray_count + self.shadow_ray_count)
 
 
-INTEGRATOR = {"direct": 0, "ao": 1}  # PRB_INTEGRATOR_*
+INTEGRATOR = {"direct": 0, "ao": 1, "visualfeedback": 2}  # PRB_INTEGRATOR_*
+# PRB_VF_*: what the colour of a 'visualfeedback' pixel shows
+VF_MODES = {"colored_entity_id": 0, "colored_material_id": 1, "colored_emission_id": 2, "colored_primitive_id": 3, "parameter": 4,
+            "inside": 5, "ndotv": 6}
 
 
 class Integrator(C.Structure):
+    """prb_integrator; its second word is a union: sample_count ('ao') or mode ('visualfeedback')"""
     _fields_ = [("type", C.c_uint32), ("sample_count", C.c_uint32)]
+    mode = property(lambda self: self.sample_count, lambda self, v: setattr(self, "sample_count", v))
 
 
 class MaterialQuery(C.Structure):
@@ -398,17 +403,20 @@ class Context:
         self.scene = scene
         rec = scene.integrator
         if rec.type != INTEGRATOR["direct"]:  # 'direct' is what prb_upload_scene leaves selected
-            self.set_integrator(rec.type, rec.sample_count)
+            self._chk(self._lib.prb_set_integrator(self._h, C.byref(rec)), "prb_set_integrator")
 
-    def set_integrator(self, integrator, sample_count=0):
-        """integrator: "direct" / "ao" or a PRB_INTEGRATOR_* value; sample_count: occlusion rays per sample ('ao')"""
+    def set_integrator(self, integrator, sample_count=0, mode="colored_entity_id"):
+        """integrator: "direct" / "ao" / "visualfeedback" or a PRB_INTEGRATOR_* value; sample_count: occlusion rays per sample
+        ('ao'); mode: a VF_MODES name or PRB_VF_* value ('visualfeedback')"""
         t = INTEGRATOR[integrator] if isinstance(integrator, str) else int(integrator)
         rec = Integrator(t, int(sample_count))
+        if t == INTEGRATOR["visualfeedback"]:
+            rec.mode = VF_MODES[mode] if isinstance(mode, str) else int(mode)
         self._chk(self._lib.prb_set_integrator(self._h, C.byref(rec)), "prb_set_integrator")
 
     @property
     def integrator(self):
-        """(type, sample_count) of the integrator prb_render_tiles runs"""
+        """(type, sample_count or mode) of the integrator prb_render_tiles runs"""
         rec = Integrator()
         self._chk(self._lib.prb_get_integrator(self._h, C.byref(rec)), "prb_get_integrator")
         return int(rec.type), int(rec.sample_count)

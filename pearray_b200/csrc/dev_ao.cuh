@@ -31,14 +31,13 @@ struct AOState {
 	uint32_t parity;	  // iteration & 1: which CNT_AO_HITS counter is in use
 };
 
-// the render starts: iteration counters, and for a render from scratch the per-pixel sums (as k_init_slots does for 'direct')
-__global__ void __launch_bounds__(128) k_ao_begin(WFState W, AOState A)
+// the render of an integrator whose samples end at the first hit ('ao', 'vf') starts: iteration counters, and for a render from
+// scratch the per-pixel sums (as k_init_slots does for 'direct')
+PRB_DEV void beginFirstHitRender(const WFState& W, uint32_t slot)
 {
-	const uint32_t slot = blockIdx.x * blockDim.x + threadIdx.x;
 	if (slot < W.nSlots) {
 		const uint32_t pix = W.pixel[slot];
 		W.iter[slot]		= W.firstIter;
-		A.occluded[slot]	= 0;
 		if (W.firstIter == 0) {
 			W.sampleCount[pix] = 0;
 			W.feedback[pix]	   = 0;
@@ -60,8 +59,18 @@ __global__ void __launch_bounds__(128) k_ao_begin(WFState W, AOState A)
 		}
 	}
 	if (blockIdx.x == 0 && threadIdx.x == 0) {
-		W.counters[CNT_END_ITER]	= W.endIter;
-		W.counters[CNT_WORK]		= 0;
+		W.counters[CNT_END_ITER] = W.endIter;
+		W.counters[CNT_WORK]	 = 0;
+	}
+}
+
+__global__ void __launch_bounds__(128) k_ao_begin(WFState W, AOState A)
+{
+	const uint32_t slot = blockIdx.x * blockDim.x + threadIdx.x;
+	beginFirstHitRender(W, slot);
+	if (slot < W.nSlots)
+		A.occluded[slot] = 0;
+	if (blockIdx.x == 0 && threadIdx.x == 0) {
 		W.counters[CNT_AO_HITS]		= 0;
 		W.counters[CNT_AO_HITS + 1] = 0;
 	}

@@ -1,6 +1,6 @@
 // C-ABI implementation (include/prb200_abi.h) over the CUDA kernels.  sm_100a only; no CPU fallback: every
 // entry point fails with PRB_ERR_NO_DEVICE / PRB_ERR_CUDA when no B200-class device is usable.
-#include "dev_ao.cuh"
+#include "dev_vf.cuh"
 
 #include <dlfcn.h>
 
@@ -156,12 +156,13 @@ struct prb_ctx {
 	uint64_t stageLaunches[PRB_STAGE__COUNT] = {};
 	// the integrator prb_render_tiles runs (prb_set_integrator; prb_upload_scene resets it to 'direct')
 	prb_integrator integrator{ PRB_INTEGRATOR_DIRECT, 0 };
-	// 'ao': per-slot state of the running sample, the hit list, the jump-ahead table, and a graph of its own
+	// 'ao': per-slot state of the running sample, the hit list, the jump-ahead table
 	DBuf<uint64_t> aoRng, aoJump;
 	DBuf<uint32_t> aoOccluded, aoHits;
 	int gridAOSmall = 148 * 4, gridAO = 148 * 4; // persistent k_ao_occlusion grids
-	cudaGraphExec_t aoGraph = nullptr;
-	uint64_t aoGraphKey[6] = {};
+	// 'ao' and 'vf': the graph of ITERS_PER_GRAPH iterations (renderFirstHit) and what it was captured for
+	cudaGraphExec_t firstHitGraph = nullptr;
+	uint64_t firstHitGraphKey[7] = {};
 };
 
 template <int KIND>
@@ -254,8 +255,8 @@ void prb_destroy(prb_ctx* c)
 	for (cudaGraphExec_t& g : c->graphExec)
 		if (g)
 			cudaGraphExecDestroy(g);
-	if (c->aoGraph)
-		cudaGraphExecDestroy(c->aoGraph);
+	if (c->firstHitGraph)
+		cudaGraphExecDestroy(c->firstHitGraph);
 	c->aoRng.release();
 	c->aoJump.release();
 	c->aoOccluded.release();
@@ -955,11 +956,85 @@ static WFState makeWF(prb_ctx* c, uint32_t first, uint32_t count)
 	return W;
 }
 
-// 'ao': exactly iteration_count iterations of one sample per slot (k_ao_primary, k_ao_occlusion, k_ao_fold), ITERS_PER_GRAPH to a
-// CUDA graph; the kernels of the iterations past the end of the range find every slot done (CNT_END_ITER) and return at once
-static prb_status renderAO(prb_ctx* c, uint32_t first, uint32_t count)
+// The integrators whose samples end at the first hit ('ao', 'vf'): exactly iteration_count iterations of one sample per slot,
+// ITERS_PER_GRAPH to a CUDA graph; the kernels of the iterations past the end of the range find every slot done (CNT_END_ITER)
+// and return at once.  begin() enqueues the per-render start after the counters are cleared; launch(parity, k) enqueues kernel k
+// of an iteration, which counts as stage[k] under profiling; key names everything the captured launches depend on.
+extern "C++" {
+template <class Begin, class Launch>
+static prb_status renderFirstHit(prb_ctx* c, uint32_t first, uint32_t count, int kernels, const int* stage, const uint64_t (&key)[7],
+								 const Begin& begin, const Launch& launch)
 {
 	constexpr int ITERS_PER_GRAPH = 8;
+	cudaStream_t s	 = c->stream;
+	c->lastFirstIter = first;
+	c->lastEndIter	 = first + count;
+	CU(cudaEventRecord(c->evA, s));
+	CU(cudaMemsetAsync(c->counters.p, 0, CNT__COUNT * sizeof(uint32_t), s));
+	begin();
+	CU(cudaGetLastError());
+	const uint32_t rounds = (count + ITERS_PER_GRAPH - 1) / ITERS_PER_GRAPH;
+	if (c->profiling) { // the same launches without graph replay, each bracketed by an event pair
+		while (c->profEvents.size() < 2 * (size_t)kernels) {
+			cudaEvent_t ev;
+			CU(cudaEventCreate(&ev));
+			c->profEvents.push_back(ev);
+		}
+		for (uint32_t r = 0; r < rounds * ITERS_PER_GRAPH; ++r)
+			for (int k = 0; k < kernels; ++k) {
+				CU(cudaEventRecord(c->profEvents[2 * k], s));
+				launch(r & 1u, k);
+				CU(cudaEventRecord(c->profEvents[2 * k + 1], s));
+				CU(cudaGetLastError());
+				CU(cudaEventSynchronize(c->profEvents[2 * k + 1]));
+				float ms = 0;
+				CU(cudaEventElapsedTime(&ms, c->profEvents[2 * k], c->profEvents[2 * k + 1]));
+				c->stageMs[stage[k]] += ms;
+				c->stageLaunches[stage[k]] += 1;
+			}
+	} else {
+		// the kernels read the iteration range from device memory, so one graph serves every call until the key changes
+		if (!c->firstHitGraph || std::memcmp(key, c->firstHitGraphKey, sizeof(key)) != 0) {
+			if (c->firstHitGraph) {
+				cudaGraphExecDestroy(c->firstHitGraph);
+				c->firstHitGraph = nullptr;
+			}
+			cudaGraph_t graph = nullptr;
+			cudaError_t be	  = cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal);
+			if (be == cudaSuccess)
+				for (int r = 0; r < ITERS_PER_GRAPH; ++r)
+					for (int k = 0; k < kernels; ++k)
+						launch((uint32_t)(r & 1), k);
+			const cudaError_t ce = be == cudaSuccess ? cudaGetLastError() : be;
+			const cudaError_t ee = be == cudaSuccess ? cudaStreamEndCapture(s, &graph) : be;
+			if (ce != cudaSuccess || ee != cudaSuccess) {
+				if (graph)
+					cudaGraphDestroy(graph);
+				return fail(PRB_ERR_CUDA, std::string("graph capture failed: ") + cudaGetErrorString(ce != cudaSuccess ? ce : ee));
+			}
+			const cudaError_t ie = cudaGraphInstantiate(&c->firstHitGraph, graph, 0);
+			cudaGraphDestroy(graph);
+			if (ie != cudaSuccess) {
+				c->firstHitGraph = nullptr;
+				return fail(PRB_ERR_CUDA, std::string("graph instantiation failed: ") + cudaGetErrorString(ie));
+			}
+			std::memcpy(c->firstHitGraphKey, key, sizeof(key));
+		}
+		for (uint32_t r = 0; r < rounds; ++r)
+			CU(cudaGraphLaunch(c->firstHitGraph, s));
+	}
+	c->kernelLaunches += 1 + (uint64_t)kernels * ITERS_PER_GRAPH * rounds;
+	c->wavefrontIterations += (uint64_t)ITERS_PER_GRAPH * rounds;
+	CU(cudaEventRecord(c->evB, s));
+	CU(cudaEventSynchronize(c->evB));
+	CU(cudaEventElapsedTime(&c->lastMs, c->evA, c->evB));
+	return PRB_OK;
+}
+}
+
+// 'ao': k_ao_primary, k_ao_occlusion, k_ao_fold per iteration
+static prb_status renderAO(prb_ctx* c, uint32_t first, uint32_t count)
+{
 	const uint32_t n = c->integrator.sample_count;
 	if ((uint64_t)c->nSlots * n > 0xFFFFFFFFull)
 		return fail(PRB_ERR_UNSUPPORTED, "'ao': owned pixels x sample_count exceeds the 32-bit work counter");
@@ -970,8 +1045,6 @@ static prb_status renderAO(prb_ctx* c, uint32_t first, uint32_t count)
 	const WFState W	 = makeWF(c, first, count);
 	AOState A{ c->aoRng.p, c->aoOccluded.p, c->aoHits.p, c->aoJump.p, n, 0 };
 	const int blocks = (int)((c->nSlots + 127) / 128);
-	c->lastFirstIter = first;
-	c->lastEndIter	 = first + count;
 	auto launch		 = [&](uint32_t parity, int kernel) { // kernel 0: primary, 1: occlusion, 2: fold
 		A.parity = parity;
 		if (kernel == 0) {
@@ -988,70 +1061,28 @@ static prb_status renderAO(prb_ctx* c, uint32_t first, uint32_t count)
 			k_ao_fold<<<blocks, 128, 0, s>>>(c->S, W, A);
 		}
 	};
-	CU(cudaEventRecord(c->evA, s));
-	CU(cudaMemsetAsync(c->counters.p, 0, CNT__COUNT * sizeof(uint32_t), s));
-	k_ao_begin<<<blocks, 128, 0, s>>>(W, A);
-	CU(cudaGetLastError());
-	const uint32_t rounds = (count + ITERS_PER_GRAPH - 1) / ITERS_PER_GRAPH;
-	if (c->profiling) { // the same launches without graph replay, each bracketed by an event pair: primary + occlusion TRACE, fold SHADE
-		while (c->profEvents.size() < 6) {
-			cudaEvent_t ev;
-			CU(cudaEventCreate(&ev));
-			c->profEvents.push_back(ev);
-		}
-		for (uint32_t r = 0; r < rounds * ITERS_PER_GRAPH; ++r)
-			for (int k = 0; k < 3; ++k) {
-				CU(cudaEventRecord(c->profEvents[2 * k], s));
-				launch(r & 1u, k);
-				CU(cudaEventRecord(c->profEvents[2 * k + 1], s));
-				CU(cudaGetLastError());
-				CU(cudaEventSynchronize(c->profEvents[2 * k + 1]));
-				float ms = 0;
-				CU(cudaEventElapsedTime(&ms, c->profEvents[2 * k], c->profEvents[2 * k + 1]));
-				const int stage = k == 2 ? PRB_STAGE_SHADE : PRB_STAGE_TRACE;
-				c->stageMs[stage] += ms;
-				c->stageLaunches[stage] += 1;
-			}
-	} else {
-		// the kernels read the iteration range from device memory, so one graph serves every call until the scene, the slot
-		// buffers, the trace variant or sample_count change
-		const uint64_t key[6] = { c->stateVersion, (uint64_t)(c->smallScene ? 1u : 0u) | (c->wantAOV ? 2u : 0u), n,
+	static const int stage[3] = { PRB_STAGE_TRACE, PRB_STAGE_TRACE, PRB_STAGE_SHADE };
+	const uint64_t key[7]	  = { PRB_INTEGRATOR_AO, c->stateVersion, (uint64_t)(c->smallScene ? 1u : 0u) | (c->wantAOV ? 2u : 0u), n,
 								  (uint64_t)(uintptr_t)A.jump, (uint64_t)(uintptr_t)A.rng, (uint64_t)(uintptr_t)A.hits };
-		if (!c->aoGraph || std::memcmp(key, c->aoGraphKey, sizeof(key)) != 0) {
-			if (c->aoGraph) {
-				cudaGraphExecDestroy(c->aoGraph);
-				c->aoGraph = nullptr;
-			}
-			cudaGraph_t graph = nullptr;
-			cudaError_t be	  = cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal);
-			if (be == cudaSuccess)
-				for (int r = 0; r < ITERS_PER_GRAPH; ++r)
-					for (int k = 0; k < 3; ++k)
-						launch((uint32_t)(r & 1), k);
-			const cudaError_t ce = be == cudaSuccess ? cudaGetLastError() : be;
-			const cudaError_t ee = be == cudaSuccess ? cudaStreamEndCapture(s, &graph) : be;
-			if (ce != cudaSuccess || ee != cudaSuccess) {
-				if (graph)
-					cudaGraphDestroy(graph);
-				return fail(PRB_ERR_CUDA, std::string("graph capture failed: ") + cudaGetErrorString(ce != cudaSuccess ? ce : ee));
-			}
-			const cudaError_t ie = cudaGraphInstantiate(&c->aoGraph, graph, 0);
-			cudaGraphDestroy(graph);
-			if (ie != cudaSuccess) {
-				c->aoGraph = nullptr;
-				return fail(PRB_ERR_CUDA, std::string("graph instantiation failed: ") + cudaGetErrorString(ie));
-			}
-			std::memcpy(c->aoGraphKey, key, sizeof(key));
-		}
-		for (uint32_t r = 0; r < rounds; ++r)
-			CU(cudaGraphLaunch(c->aoGraph, s));
-	}
-	c->kernelLaunches += 1 + 3ull * ITERS_PER_GRAPH * rounds;
-	c->wavefrontIterations += (uint64_t)ITERS_PER_GRAPH * rounds;
-	CU(cudaEventRecord(c->evB, s));
-	CU(cudaEventSynchronize(c->evB));
-	CU(cudaEventElapsedTime(&c->lastMs, c->evA, c->evB));
-	return PRB_OK;
+	return renderFirstHit(c, first, count, 3, stage, key, [&] { k_ao_begin<<<blocks, 128, 0, s>>>(W, A); }, launch);
+}
+
+// 'vf': k_vf per iteration
+static prb_status renderVF(prb_ctx* c, uint32_t first, uint32_t count)
+{
+	cudaStream_t s		= c->stream;
+	const WFState W		= makeWF(c, first, count);
+	const uint32_t mode = c->integrator.mode;
+	const int blocks	= (int)((c->nSlots + 127) / 128);
+	auto launch			= [&](uint32_t, int) {
+		if (c->smallScene)
+			k_vf<true><<<blocks, 128, 0, s>>>(c->S, W, mode);
+		else
+			k_vf<false><<<blocks, 128, 0, s>>>(c->S, W, mode);
+	};
+	static const int stage[1] = { PRB_STAGE_TRACE };
+	const uint64_t key[7] = { PRB_INTEGRATOR_VF, c->stateVersion, (uint64_t)(c->smallScene ? 1u : 0u) | (c->wantAOV ? 2u : 0u), mode, 0, 0, 0 };
+	return renderFirstHit(c, first, count, 1, stage, key, [&] { k_vf_begin<<<blocks, 128, 0, s>>>(W); }, launch);
 }
 
 prb_status prb_set_integrator(prb_ctx* c, const prb_integrator* in)
@@ -1060,8 +1091,14 @@ prb_status prb_set_integrator(prb_ctx* c, const prb_integrator* in)
 		return fail(PRB_ERR_INVALID_ARG, "null argument");
 	if (!c->haveScene)
 		return fail(PRB_ERR_NO_SCENE, "no scene uploaded");
-	if (in->type != PRB_INTEGRATOR_DIRECT && in->type != PRB_INTEGRATOR_AO)
+	if (in->type != PRB_INTEGRATOR_DIRECT && in->type != PRB_INTEGRATOR_AO && in->type != PRB_INTEGRATOR_VF)
 		return fail(PRB_ERR_INVALID_ARG, "unknown integrator type " + std::to_string(in->type));
+	if (in->type == PRB_INTEGRATOR_VF) {
+		if (in->mode >= PRB_VF__COUNT)
+			return fail(PRB_ERR_INVALID_ARG, "unknown 'vf' mode " + std::to_string(in->mode));
+		if (c->S.nLPE)
+			return fail(PRB_ERR_UNSUPPORTED, "'vf' does not fill light path expression channels");
+	}
 	if (in->type == PRB_INTEGRATOR_AO) {
 		if (in->sample_count == 0)
 			return fail(PRB_ERR_INVALID_ARG, "'ao' needs sample_count >= 1");
@@ -1105,6 +1142,8 @@ prb_status prb_render_tiles(prb_ctx* c, const prb_tile* tiles, size_t n_tiles, u
 		return st;
 	if (c->integrator.type == PRB_INTEGRATOR_AO)
 		return renderAO(c, first_iteration, iteration_count);
+	if (c->integrator.type == PRB_INTEGRATOR_VF)
+		return renderVF(c, first_iteration, iteration_count);
 	cudaStream_t s = c->stream;
 	const WFState W	 = makeWF(c, first_iteration, iteration_count);
 	const int blocks = (int)((c->nSlots + 127) / 128);

@@ -546,7 +546,7 @@ void SceneLoader::addIntegrator(const DL::DataGroup& group, SceneLoadContext& ct
 		return;
 	auto fac = ctx.environment()->integratorManager.getFactory(type);
 	if (!fac) {
-		PR_LOG(L_ERROR) << "[Loader] Unknown integrator type " << type << " (the device path has the 'direct' path tracer and 'ao')" << std::endl;
+		PR_LOG(L_ERROR) << "[Loader] Unknown integrator type " << type << " (the device path has the 'direct' path tracer, 'ao' and 'visualfeedback')" << std::endl;
 		return;
 	}
 	ctx.parameters() = populateObjectParameters(group, ctx);

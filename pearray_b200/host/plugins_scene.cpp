@@ -1262,6 +1262,70 @@ public:
 	std::string specification(const std::string&) const override { return "AO / Ambient Occlusion: sample_count (10)"; }
 };
 
+// ------------------------------------------------------------------ 'visualfeedback' integrator -> device
+// reference plugins/main/integrators/visualfeedback.cpp: one parameter, mode (what the colour of a pixel shows, default
+// colored_entity_id; the names are listed in vfModeNames).  The tiles go to prb_render_tiles like 'direct'; RenderContext
+// selects the kernel with prb_set_integrator.
+static const char* const vfModeNames[PRB_VF__COUNT] = { "colored_entity_id", "colored_material_id", "colored_emission_id",
+														 "colored_primitive_id", "parameter", "inside", "ndotv" }; // PRB_VF_*
+class IntVF : public IIntegrator {
+public:
+	explicit IntVF(uint32 mode)
+		: mMode(mode)
+	{
+	}
+	std::shared_ptr<IIntegratorInstance> createThreadInstance(RenderContext*, size_t) override { return std::make_shared<IntDirectInstance>(); }
+	void describe(prb_settings& s) const override
+	{ // no path beyond the first hit, no light sampling
+		s.max_ray_depth		 = 1;
+		s.soft_max_ray_depth = 1;
+		s.do_nee = s.do_direct = s.emissive_scatter = 0;
+	}
+	prb_integrator deviceIntegrator() const override
+	{
+		prb_integrator r{};
+		r.type = PRB_INTEGRATOR_VF;
+		r.mode = mMode;
+		return r;
+	}
+
+private:
+	uint32 mMode;
+};
+class IntVFFactory : public IIntegratorFactory {
+public:
+	explicit IntVFFactory(uint32 mode)
+		: mMode(mode)
+	{
+	}
+	std::shared_ptr<IIntegrator> createInstance() const override { return std::make_shared<IntVF>(mMode); }
+
+private:
+	uint32 mMode;
+};
+class IntVFFactoryFactory : public IIntegratorPlugin {
+public:
+	std::shared_ptr<IIntegratorFactory> create(const std::string&, const SceneLoadContext& ctx) override
+	{
+		std::string mode = ctx.parameters().getString("mode", vfModeNames[PRB_VF_ENTITY_ID]);
+		std::transform(mode.begin(), mode.end(), mode.begin(), ::tolower);
+		for (uint32 m = 0; m < PRB_VF__COUNT; ++m)
+			if (mode == vfModeNames[m])
+				return std::make_shared<IntVFFactory>(m);
+		PR_LOG(L_ERROR) << "[visualfeedback] Unknown mode " << mode << std::endl;
+		return nullptr;
+	}
+	const std::vector<std::string>& getNames() const override
+	{
+		static const std::vector<std::string> names({ "visualfeedback", "vf" });
+		return names;
+	}
+	std::string specification(const std::string&) const override
+	{
+		return "VF / Visual Feedback: mode colored_entity_id|colored_material_id|colored_emission_id|colored_primitive_id|parameter|inside|ndotv (colored_entity_id)";
+	}
+};
+
 void registerScenePlugins(std::vector<std::shared_ptr<IPlugin>>& out)
 {
 	out.push_back(std::make_shared<MeshEntityPlugin>());
@@ -1286,5 +1350,6 @@ void registerScenePlugins(std::vector<std::shared_ptr<IPlugin>>& out)
 	out.push_back(std::make_shared<AGHSpectralMapperPlugin>());
 	out.push_back(std::make_shared<IntDirectFactoryFactory>());
 	out.push_back(std::make_shared<IntAOFactoryFactory>());
+	out.push_back(std::make_shared<IntVFFactoryFactory>());
 }
 } // namespace PR
