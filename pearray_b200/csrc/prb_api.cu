@@ -32,10 +32,20 @@ prb_status fail(prb_status code, const std::string& msg)
 			return fail(PRB_ERR_CUDA, std::string(#x) + ": " + cudaGetErrorString(e_));                           \
 	} while (0)
 
+// a device buffer that frees itself; movable, not copyable
 template <typename T>
 struct DBuf {
 	T* p	 = nullptr;
 	size_t n = 0;
+	DBuf() = default;
+	DBuf(DBuf&& o) noexcept { *this = std::move(o); }
+	DBuf& operator=(DBuf&& o) noexcept
+	{
+		std::swap(p, o.p);
+		std::swap(n, o.n);
+		return *this;
+	}
+	~DBuf() { release(); }
 	cudaError_t alloc(size_t count)
 	{
 		if (count <= n && p)
@@ -61,12 +71,72 @@ struct DBuf {
 		n = 0;
 	}
 };
+
+// one CUDA runtime handle (stream, event, graph exec, pinned block), passed to Destroy when the owner goes; movable, not copyable
+template <typename H, auto Destroy>
+struct Owned {
+	H h = nullptr;
+	Owned() = default;
+	explicit Owned(H handle) : h(handle) {}
+	Owned(Owned&& o) noexcept { std::swap(h, o.h); }
+	~Owned() { reset(); }
+	void reset()
+	{
+		if (h)
+			Destroy(h);
+		h = nullptr;
+	}
+	operator H() const { return h; }
+};
+using Event = Owned<cudaEvent_t, cudaEventDestroy>;
+
+// an instantiated CUDA graph and the key naming everything its captured launches depend on
+struct CachedGraph {
+	Owned<cudaGraphExec_t, cudaGraphExecDestroy> exec;
+	uint64_t key[7] = {};
+	// re-captures what enqueue() launches on s unless the graph was captured for `k`
+	template <class Enqueue>
+	prb_status update(cudaStream_t s, const uint64_t (&k)[7], const Enqueue& enqueue)
+	{
+		if (exec && std::memcmp(k, key, sizeof(key)) == 0)
+			return PRB_OK;
+		exec.reset();
+		cudaGraph_t graph = nullptr;
+		cudaError_t be	  = cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal);
+		if (be == cudaSuccess)
+			enqueue();
+		const cudaError_t ce = be == cudaSuccess ? cudaGetLastError() : be;
+		const cudaError_t ee = be == cudaSuccess ? cudaStreamEndCapture(s, &graph) : be;
+		if (ce != cudaSuccess || ee != cudaSuccess) {
+			if (graph)
+				cudaGraphDestroy(graph);
+			return fail(PRB_ERR_CUDA, std::string("graph capture failed: ") + cudaGetErrorString(ce != cudaSuccess ? ce : ee));
+		}
+		const cudaError_t ie = cudaGraphInstantiate(&exec.h, graph, 0);
+		cudaGraphDestroy(graph);
+		if (ie != cudaSuccess) {
+			exec.h = nullptr;
+			return fail(PRB_ERR_CUDA, std::string("graph instantiation failed: ") + cudaGetErrorString(ie));
+		}
+		std::memcpy(key, k, sizeof(key));
+		return PRB_OK;
+	}
+};
 } // namespace
 
+// Every device buffer and handle below frees itself.  Members go in reverse order of declaration, so the stream, declared
+// first, outlives everything that was enqueued on it.
 struct prb_ctx {
 	int device = 0;
-	cudaStream_t stream = nullptr;
-	cudaEvent_t evA = nullptr, evB = nullptr, evT0 = nullptr, evT1 = nullptr;
+	Owned<cudaStream_t, cudaStreamDestroy> stream;
+	Event evA, evB, evT0, evT1;
+	~prb_ctx()
+	{
+		cudaSetDevice(device);
+		if (stream)
+			cudaStreamSynchronize(stream);
+		prb_comm_destroy(this);
+	}
 	int smCount = 148;
 	bool allLambert = false;	 // every material is PRB_MAT_DIFFUSE: k_shade with the Lambert code inline
 	bool hasImageNodes = false;	 // some node is an image texture: no kernel with the Lambert code inline (leaf-only node evaluation)
@@ -131,7 +201,7 @@ struct prb_ctx {
 	DBuf<float> lpeFilm; // n_lpe films of npix * 3 floats
 	std::vector<prb_tile> cachedTiles;
 	uint32_t nSlots = 0;
-	uint32_t* hostCounters = nullptr; // pinned
+	Owned<uint32_t*, cudaFreeHost> hostCounters; // pinned
 	// generic scratch for the host-pointer entry points
 	DBuf<float> scratchF;
 	DBuf<uint32_t> scratchU;
@@ -143,15 +213,15 @@ struct prb_ctx {
 	float lastMs = 0;
 	// the wavefront graph (ITERS_PER_GRAPH x k_trace, k_shade, k_regen) is instantiated once and replayed by every
 	// prb_render_tiles call until something baked into its kernel parameters changes (scene, slot buffers, variant)
-	cudaGraphExec_t graphExec[2] = { nullptr, nullptr }; // [staged]
-	uint64_t graphKey[2] = { 0, 0 }, stateVersion = 1; // stateVersion: bumped whenever the scene or the slot buffers change
+	CachedGraph directGraph[2]; // [staged]
+	uint64_t stateVersion = 1; // bumped whenever the scene or the slot buffers change
 	bool wantAOV = true;
 	bool persistentTrace = true; // k_trace (persistent threads) vs k_trace_static, chosen per scene in prb_upload_scene
 	bool smallScene = false;	 // k_trace_small: a tiny scene traced from shared memory, no BVH
 	DBuf<uint4> small;
 	// per-stage profiling (prb_set_profiling)
 	bool profiling = false;
-	std::vector<cudaEvent_t> profEvents; // pairs
+	std::vector<Event> profEvents; // pairs
 	float stageMs[PRB_STAGE__COUNT] = {};
 	uint64_t stageLaunches[PRB_STAGE__COUNT] = {};
 	// the integrator prb_render_tiles runs (prb_set_integrator; prb_upload_scene resets it to 'direct')
@@ -161,9 +231,19 @@ struct prb_ctx {
 	DBuf<uint32_t> aoOccluded, aoHits;
 	int gridAOSmall = 148 * 4, gridAO = 148 * 4; // persistent k_ao_occlusion grids
 	// 'ao' and 'vf': the graph of ITERS_PER_GRAPH iterations (renderFirstHit) and what it was captured for
-	cudaGraphExec_t firstHitGraph = nullptr;
-	uint64_t firstHitGraphKey[7] = {};
+	CachedGraph firstHitGraph;
 };
+
+// grows the pool of profiling events to at least n
+static prb_status reserveProfEvents(prb_ctx* c, size_t n)
+{
+	while (c->profEvents.size() < n) {
+		cudaEvent_t ev;
+		CU(cudaEventCreate(&ev));
+		c->profEvents.emplace_back(ev);
+	}
+	return PRB_OK;
+}
 
 template <int KIND>
 static void launchStageKernels(prb_ctx* c, const WFState& W, uint32_t queue, cudaStream_t s)
@@ -209,17 +289,12 @@ prb_status prb_create(int device, prb_ctx** out)
 	auto* c		= new prb_ctx();
 	c->device	= device;
 	c->smCount	= prop.multiProcessorCount;
-	cudaError_t e = cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking);
+	cudaError_t e = cudaStreamCreateWithFlags(&c->stream.h, cudaStreamNonBlocking);
+	for (Event* ev : { &c->evA, &c->evB, &c->evT0, &c->evT1 })
+		if (e == cudaSuccess)
+			e = cudaEventCreate(&ev->h);
 	if (e == cudaSuccess)
-		e = cudaEventCreate(&c->evA);
-	if (e == cudaSuccess)
-		e = cudaEventCreate(&c->evB);
-	if (e == cudaSuccess)
-		e = cudaEventCreate(&c->evT0);
-	if (e == cudaSuccess)
-		e = cudaEventCreate(&c->evT1);
-	if (e == cudaSuccess)
-		e = cudaMallocHost(&c->hostCounters, CNT__COUNT * sizeof(uint32_t));
+		e = cudaMallocHost(&c->hostCounters.h, CNT__COUNT * sizeof(uint32_t));
 	if (e == cudaSuccess)
 		e = c->stats.alloc(ST__COUNT);
 	if (e == cudaSuccess)
@@ -246,64 +321,7 @@ prb_status prb_create(int device, prb_ctx** out)
 	return PRB_OK;
 }
 
-void prb_destroy(prb_ctx* c)
-{
-	if (!c)
-		return;
-	cudaSetDevice(c->device);
-	cudaStreamSynchronize(c->stream);
-	for (cudaGraphExec_t& g : c->graphExec)
-		if (g)
-			cudaGraphExecDestroy(g);
-	if (c->firstHitGraph)
-		cudaGraphExecDestroy(c->firstHitGraph);
-	c->aoRng.release();
-	c->aoJump.release();
-	c->aoOccluded.release();
-	c->aoHits.release();
-	prb_comm_destroy(c);
-	c->reduceF.release();
-	c->reduceU.release();
-	DBuf<uint32_t>* ub[] = { &c->entityMaterials, &c->faceIndices, &c->faceSlots, &c->tlasRefs, &c->sampleCount, &c->feedback, &c->pixel, &c->iter, &c->flagsDepth,
-							 &c->slotState, &c->counters, &c->regenList, &c->activeList, &c->neeList, &c->scatterList, &c->scratchU };
-	for (auto* b : ub)
-		b->release();
-	DBuf<float>* fb[] = { &c->vertices, &c->normals, &c->uvs, &c->lightCDF, &c->pool, &c->rrProb, &c->filmMean, &c->filmTmp, &c->aov, &c->aovExt, &c->varMean, &c->varVar, &c->hitT, &c->scratchF };
-	for (auto* b : fb)
-		b->release();
-	DBuf<float4>* f4[] = { &c->bvhTris, &c->rayO, &c->rayD, &c->wvl, &c->thr, &c->pathPDF, &c->prevPDF, &c->wvlPDF, &c->lastPos, &c->shO, &c->shD, &c->shXYZ, &c->iterXYZ, &c->prevAcc, &c->vxP, &c->vxN, &c->vxNx, &c->vxNy, &c->vxD };
-	for (auto* b : f4)
-		b->release();
-	c->nodes.release();
-	c->materials.release();
-	c->emissions.release();
-	c->entities.release();
-	c->meshes.release();
-	c->lights.release();
-	c->bvhNodes.release();
-	c->rng.release();
-	c->stats.release();
-	c->hit.release();
-	c->lpeTables.release();
-	c->lpeState.release();
-	c->lpeAcc.release();
-	c->lpePrev.release();
-	c->lpeFilm.release();
-	c->scratchB.release();
-	c->small.release();
-	c->scratchQ.release();
-	c->scratchR.release();
-	if (c->hostCounters)
-		cudaFreeHost(c->hostCounters);
-	for (cudaEvent_t ev : c->profEvents)
-		cudaEventDestroy(ev);
-	cudaEventDestroy(c->evA);
-	cudaEventDestroy(c->evB);
-	cudaEventDestroy(c->evT0);
-	cudaEventDestroy(c->evT1);
-	cudaStreamDestroy(c->stream);
-	delete c;
-}
+void prb_destroy(prb_ctx* c) { delete c; }
 
 // number of BVH8 levels below (and including) `root`; 0 when an index is out of range or the tree is deeper than `limit`
 static uint32_t bvhLevels(const prb_scene_desc* d, uint32_t root, uint32_t limit)
@@ -975,11 +993,9 @@ static prb_status renderFirstHit(prb_ctx* c, uint32_t first, uint32_t count, int
 	CU(cudaGetLastError());
 	const uint32_t rounds = (count + ITERS_PER_GRAPH - 1) / ITERS_PER_GRAPH;
 	if (c->profiling) { // the same launches without graph replay, each bracketed by an event pair
-		while (c->profEvents.size() < 2 * (size_t)kernels) {
-			cudaEvent_t ev;
-			CU(cudaEventCreate(&ev));
-			c->profEvents.push_back(ev);
-		}
+		const prb_status ps = reserveProfEvents(c, 2 * (size_t)kernels);
+		if (ps != PRB_OK)
+			return ps;
 		for (uint32_t r = 0; r < rounds * ITERS_PER_GRAPH; ++r)
 			for (int k = 0; k < kernels; ++k) {
 				CU(cudaEventRecord(c->profEvents[2 * k], s));
@@ -994,34 +1010,15 @@ static prb_status renderFirstHit(prb_ctx* c, uint32_t first, uint32_t count, int
 			}
 	} else {
 		// the kernels read the iteration range from device memory, so one graph serves every call until the key changes
-		if (!c->firstHitGraph || std::memcmp(key, c->firstHitGraphKey, sizeof(key)) != 0) {
-			if (c->firstHitGraph) {
-				cudaGraphExecDestroy(c->firstHitGraph);
-				c->firstHitGraph = nullptr;
-			}
-			cudaGraph_t graph = nullptr;
-			cudaError_t be	  = cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal);
-			if (be == cudaSuccess)
-				for (int r = 0; r < ITERS_PER_GRAPH; ++r)
-					for (int k = 0; k < kernels; ++k)
-						launch((uint32_t)(r & 1), k);
-			const cudaError_t ce = be == cudaSuccess ? cudaGetLastError() : be;
-			const cudaError_t ee = be == cudaSuccess ? cudaStreamEndCapture(s, &graph) : be;
-			if (ce != cudaSuccess || ee != cudaSuccess) {
-				if (graph)
-					cudaGraphDestroy(graph);
-				return fail(PRB_ERR_CUDA, std::string("graph capture failed: ") + cudaGetErrorString(ce != cudaSuccess ? ce : ee));
-			}
-			const cudaError_t ie = cudaGraphInstantiate(&c->firstHitGraph, graph, 0);
-			cudaGraphDestroy(graph);
-			if (ie != cudaSuccess) {
-				c->firstHitGraph = nullptr;
-				return fail(PRB_ERR_CUDA, std::string("graph instantiation failed: ") + cudaGetErrorString(ie));
-			}
-			std::memcpy(c->firstHitGraphKey, key, sizeof(key));
-		}
+		const prb_status gs = c->firstHitGraph.update(s, key, [&] {
+			for (int r = 0; r < ITERS_PER_GRAPH; ++r)
+				for (int k = 0; k < kernels; ++k)
+					launch((uint32_t)(r & 1), k);
+		});
+		if (gs != PRB_OK)
+			return gs;
 		for (uint32_t r = 0; r < rounds; ++r)
-			CU(cudaGraphLaunch(c->firstHitGraph, s));
+			CU(cudaGraphLaunch(c->firstHitGraph.exec, s));
 	}
 	c->kernelLaunches += 1 + (uint64_t)kernels * ITERS_PER_GRAPH * rounds;
 	c->wavefrontIterations += (uint64_t)ITERS_PER_GRAPH * rounds;
@@ -1170,12 +1167,9 @@ prb_status prb_render_tiles(prb_ctx* c, const prb_tile* tiles, size_t n_tiles, u
 	};
 	if (c->profiling) {
 		// same launch sequence without graph replay, every kernel bracketed by an event pair on the context stream
-		const size_t needEvents = (size_t)ITERS_PER_GRAPH * GRAPHS_PER_POLL * PRB_STAGE__COUNT * 2;
-		while (c->profEvents.size() < needEvents) {
-			cudaEvent_t ev;
-			CU(cudaEventCreate(&ev));
-			c->profEvents.push_back(ev);
-		}
+		const prb_status ps = reserveProfEvents(c, (size_t)ITERS_PER_GRAPH * GRAPHS_PER_POLL * PRB_STAGE__COUNT * 2);
+		if (ps != PRB_OK)
+			return ps;
 		while (!finished && done < maxIters + ITERS_PER_GRAPH * GRAPHS_PER_POLL) {
 			size_t ne = 0;
 			for (int r = 0; r < ITERS_PER_GRAPH * GRAPHS_PER_POLL; ++r) {
@@ -1201,41 +1195,6 @@ prb_status prb_render_tiles(prb_ctx* c, const prb_tile* tiles, size_t n_tiles, u
 			}
 		}
 	} else {
-		// the kernels of the graph read the iteration range from device memory (CNT_END_ITER, written by k_init_slots), so one
-		// instantiated graph serves every call until the scene, the slot buffers or the kernel variant change
-		auto ensureGraph = [&](bool stagedMode) -> prb_status {
-			const uint64_t key = (c->stateVersion << 4) | (c->persistentTrace ? 1u : 0u) | (c->wantAOV ? 2u : 0u) | (c->smallScene ? 4u : 0u) | (stagedMode ? 8u : 0u);
-			cudaGraphExec_t& exec = c->graphExec[stagedMode ? 1 : 0];
-			if (exec && c->graphKey[stagedMode ? 1 : 0] == key)
-				return PRB_OK;
-			if (exec) {
-				cudaGraphExecDestroy(exec);
-				exec = nullptr;
-			}
-			const bool keep = c->staged;
-			c->staged		= stagedMode;
-			cudaGraph_t graph = nullptr;
-			cudaError_t be	  = cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal);
-			if (be == cudaSuccess)
-				for (int r = 0; r < ITERS_PER_GRAPH; ++r)
-					launchIteration(c, W, blocks, s, r);
-			c->staged = keep;
-			const cudaError_t ce = be == cudaSuccess ? cudaGetLastError() : be;
-			const cudaError_t ee = be == cudaSuccess ? cudaStreamEndCapture(s, &graph) : be;
-			if (ce != cudaSuccess || ee != cudaSuccess) {
-				if (graph)
-					cudaGraphDestroy(graph);
-				return fail(PRB_ERR_CUDA, std::string("graph capture failed: ") + cudaGetErrorString(ce != cudaSuccess ? ce : ee));
-			}
-			const cudaError_t ie = cudaGraphInstantiate(&exec, graph, 0);
-			cudaGraphDestroy(graph);
-			if (ie != cudaSuccess) {
-				exec = nullptr;
-				return fail(PRB_ERR_CUDA, std::string("graph instantiation failed: ") + cudaGetErrorString(ie));
-			}
-			c->graphKey[stagedMode ? 1 : 0] = key;
-			return PRB_OK;
-		};
 		// Undecided contexts time poll intervals in the order single, staged, staged, single (the number of live paths falls
 		// slowly over a render; the symmetric order cancels that drift) and keep the faster path from then on.  Both leave the
 		// same wavefront state behind every iteration, so they can alternate freely.
@@ -1243,14 +1202,24 @@ prb_status prb_render_tiles(prb_ctx* c, const prb_tile* tiles, size_t n_tiles, u
 		while (!finished && done < maxIters + ITERS_PER_GRAPH * GRAPHS_PER_POLL) {
 			const bool tuning = c->stagedAuto && c->tuneStep < 4;
 			const bool mode	  = tuning ? tuneOrder[c->tuneStep] : c->staged;
-			prb_status gs	  = ensureGraph(mode);
+			// the kernels of the graph read the iteration range from device memory (CNT_END_ITER, written by k_init_slots), so one
+			// instantiated graph serves every call until the scene, the slot buffers or the kernel variant change
+			const uint64_t key[7] = { (c->stateVersion << 4) | (c->persistentTrace ? 1u : 0u) | (c->wantAOV ? 2u : 0u) | (c->smallScene ? 4u : 0u) | (mode ? 8u : 0u) };
+			CachedGraph& graph	  = c->directGraph[mode ? 1 : 0];
+			const prb_status gs	  = graph.update(s, key, [&] {
+				const bool keep = c->staged; // the launches read the shading mode from the context
+				c->staged		= mode;
+				for (int r = 0; r < ITERS_PER_GRAPH; ++r)
+					launchIteration(c, W, blocks, s, r);
+				c->staged = keep;
+			});
 			if (gs != PRB_OK)
 				return gs;
 			cudaError_t e = cudaSuccess;
 			if (tuning)
 				e = cudaEventRecord(c->evT0, s);
 			for (int r = 0; r < GRAPHS_PER_POLL && e == cudaSuccess; ++r)
-				e = cudaGraphLaunch(c->graphExec[mode ? 1 : 0], s);
+				e = cudaGraphLaunch(graph.exec, s);
 			if (tuning && e == cudaSuccess)
 				e = cudaEventRecord(c->evT1, s);
 			done += ITERS_PER_GRAPH * GRAPHS_PER_POLL;
@@ -1656,7 +1625,6 @@ prb_status prb_film_reduce(prb_ctx** ctxs, int n, int partition)
 			}
 		}
 		CU(cudaStreamSynchronize(root->stream));
-		stage.release();
 	}
 	if (root->varMean.p && partition == PRB_PARTITION_TILES) {
 		DBuf<float> stage;
@@ -1673,15 +1641,10 @@ prb_status prb_film_reduce(prb_ctx** ctxs, int n, int partition)
 			}
 		}
 		CU(cudaStreamSynchronize(root->stream));
-		stage.release();
 	}
 	CU(cudaEventRecord(root->evB, root->stream));
 	CU(cudaEventSynchronize(root->evB));
 	CU(cudaEventElapsedTime(&root->lastReduceMs, root->evA, root->evB));
-	for (int i = 1; i < n; ++i) {
-		stageF[i].release();
-		stageU[i].release();
-	}
 	return PRB_OK;
 }
 prb_status prb_last_reduce_ms(prb_ctx* c, float* ms)
